@@ -5,7 +5,7 @@ Workload (BASELINE.json configs[1]): one "step" = one 1 s CPI @ 2 MS/s through
 WienerHopf (410 taps) -> Ambiguity (300 delay x 257 Doppler) -> Map::set_metrics ->
 CfarDetector1D -> Centroid -> Interpolate on synthetic IQ (blah2_b200/scene.py).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Contract (one JSON line on rank 0):
   value   IQ Msamples/s, whole job over all N GPUs, inputs resident in HBM (float2), CUDA-event
@@ -238,12 +238,13 @@ def dropin_leg(sc, cpis=3):
     reference's process thread drives its own (src/blah2.cpp:268-287: WienerHopf::process -> Ambiguity::process ->
     Map::set_metrics -> CfarDetector1D -> Centroid -> Interpolate on IqData deques, Map and Detection objects),
     through the same harness source that drives the reference (oracle/ref_capi.cpp compiled against the drop-in
-    headers: tests/native).  Stage times are the harness's own (the reference's stage names); the IqData fill is the
-    caller's deque traffic (blah2.cpp:254-258) and is timed apart."""
+    headers: tests/native, built into oracle/_ref beside the reference library).  Stage times are the harness's own
+    (the reference's stage names); the IqData fill is the caller's deque traffic (blah2.cpp:254-258) and is timed
+    apart."""
     import importlib.util
-    harness = os.path.join(ROOT, "tests", "native", "_build", "libdropin_harness.so")
+    harness = os.path.join(ROOT, "oracle", "_ref", "libdropin_harness.so")
     if not os.path.exists(harness):
-        return {"unavailable": "tests/native/_build/libdropin_harness.so not built (needs /root/reference headers at build time)"}
+        return {"unavailable": "oracle/_ref/libdropin_harness.so not built (needs the blah2 sources at build time)"}
     try:
         from oracle import refpath as R
         spec = importlib.util.spec_from_file_location("dropin_binding", R.__file__)
@@ -272,6 +273,24 @@ def dropin_leg(sc, cpis=3):
         return {"unavailable": f"{type(e).__name__}: {e}"}
 
 
+def dump_outputs(out_dir, res, d_map, pipe):
+    """What a caller of the timed path receives for one CPI, as DIR/<name>.npy: the device map (complex64
+    [nDoppler][nDelay], stored as float32 [..., 2] = real, imag), set_metrics' noise and max power with the skip flag,
+    the detection list ([3][nDetections]: delay, Doppler, SNR) and the map's axes."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    det = res["detections"]
+    arrays = {
+        "map": torch.view_as_real(d_map).cpu().numpy().astype(np.float32),
+        "metrics": np.array([res["noisePower"], res["maxPower"], float(res["skipped"])], dtype=np.float64),
+        "detections": np.stack([det.delay, det.doppler, det.snr]).astype(np.float64),
+        "delay": pipe.delay.astype(np.float64),
+        "doppler": pipe.doppler.astype(np.float64),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -282,7 +301,13 @@ def main():
     ap.add_argument("--eager", action="store_true", help="launch every kernel of every CPI instead of replaying the chain as a CUDA graph")
     ap.add_argument("--streams", type=int, default=6, help="CPIs in flight per GPU (independent pipelines on their own streams)")
     ap.add_argument("--no-gather", action="store_true", help="diagnostic: N > 1 without the map gather (not a bench mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (map, metrics, detections) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -418,8 +443,9 @@ def main():
     for i in range(args.steps):
         submit(i, args.steps)
     host_submit_us = (time.perf_counter() - t_host0) / args.steps * 1e6   # the submitting thread's time per CPI
+    fetched = [None] * NPIPE
     for p in reversed(range(NPIPE)):  # synchronises each stream; detections + metrics of the final CPIs on the host
-        last = pipes[p].fetch(streams[p].cuda_stream)
+        last = fetched[p] = pipes[p].fetch(streams[p].cuda_stream)
     with torch.cuda.stream(stream):
         if comm is not None:  # the last gathers (rank 0: every rank's maps have arrived) end the region
             comm.join(stream)
@@ -435,6 +461,8 @@ def main():
         count = args.steps - first
         got = recv_all[first // NPIPE].view(-1)[: world * count * cells].view(world, count, g.n_doppler_bins, g.n_delay_bins)
         gather_check = bool(torch.equal(got[0], ring[first:first + count])) and bool(torch.isfinite(torch.view_as_real(got)).all())
+    if args.dump_outputs is not None and rank == 0:   # before anything below reuses the map slots
+        dump_outputs(args.dump_outputs, fetched[(args.steps - 1) % NPIPE], dmaps[slot_of(args.steps - 1)], pipe)
 
     # ---- end to end through the host API (pinned complex128 in, complex128 map out) ----
     # Two pipelines alternate: submit_host(i) enqueues H2D + kernels + D2H, fetch(i-1) collects the

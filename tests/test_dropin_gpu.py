@@ -1,7 +1,8 @@
 """GPU: the C++ drop-in classes (blah2_b200/dropin, same names/signatures as the reference's
 src/process classes) driven through the SAME harness source as the reference
-(oracle/ref_capi.cpp compiled unchanged against our headers -> tests/native/_build), compared
-with the reference library (oracle/_ref) or, where that is absent, the numpy oracle."""
+(oracle/ref_capi.cpp compiled unchanged against our headers -> oracle/_ref/libdropin_harness.so), compared
+with the reference's stored outputs (tests/golden/dropin_ref.npz, oracle/gen_golden_live.py) and with the
+reference library (oracle/_ref) or, where that is absent, the numpy oracle."""
 import importlib.util
 import os
 
@@ -11,17 +12,25 @@ import pytest
 from blah2_b200.scene import make_scene, random_iq, Target
 from oracle import blah2_oracle as O
 from oracle import refpath as R
+from oracle.fixture import errors as fixture_errors
 
 pytestmark = pytest.mark.gpu
 
-HARNESS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "native", "_build", "libdropin_harness.so")
+HARNESS = os.path.join(os.path.dirname(R.LIB_PATH), "libdropin_harness.so")
+GEOMS = [(-10, 300, -300, 300, 2000000, 1000000, True),   # Process_Simple geometry
+         (0, 31, -20, 60, 10000, 5000, True)]             # off-centre Doppler window
+
+
+@pytest.fixture(scope="module")
+def gold():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dropin_ref.npz"))
 
 
 @pytest.fixture(scope="module")
 def D():
     """A second instance of the refpath binding, pointed at the drop-in harness."""
     if not os.path.exists(HARNESS):
-        pytest.fail(f"{HARNESS} missing: run `make -C blah2_b200/dropin && make -C tests/native` where /root/reference exists")
+        pytest.fail(f"{HARNESS} missing: run `make -C oracle dropin` where the blah2 sources are")
     spec = importlib.util.spec_from_file_location("dropin_binding", R.__file__)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
@@ -37,11 +46,15 @@ def test_constructor_getters_like_testambiguity_cpp(D):
     assert D.next_hamming(104) == 108 and D.next_hamming(3322) == 3375 and D.next_hamming(19043) == 19200
 
 
-@pytest.mark.parametrize("geom", [(-10, 300, -300, 300, 2000000, 1000000, True),   # Process_Simple geometry
-                                  (0, 31, -20, 60, 10000, 5000, True)])            # off-centre Doppler window
-def test_ambiguity_class_matches_reference_class(D, geom, relerr):
+@pytest.mark.parametrize("geom", GEOMS)
+def test_ambiguity_class_matches_reference_class(D, geom, relerr, gold):
     x, y = random_iq(geom[5], 21)
     d = D.ambiguity_process(x, y, *geom)
+    k = GEOMS.index(geom)
+    e = fixture_errors(d["map"], gold, f"amb{k}_map")
+    assert max(e) < 1e-5, e
+    assert d["leftover"] == tuple(int(v) for v in gold[f"amb{k}_leftover"])
+    assert np.max(np.abs(np.array([d["noisePower"], d["maxPower"]]) - gold[f"amb{k}_metrics"])) < 1e-3
     if R.available():
         r = R.ambiguity_process(x, y, *geom)
         ref_map, left, noise, mx = r["map"], r["leftover"], r["noisePower"], r["maxPower"]
@@ -57,9 +70,10 @@ def test_ambiguity_class_matches_reference_class(D, geom, relerr):
     assert abs(d["noisePower"] - noise) < 1e-3 and abs(d["maxPower"] - mx) < 1e-3
 
 
-def test_wienerhopf_class_matches_reference_class(D, relerr):
+def test_wienerhopf_class_matches_reference_class(D, relerr, gold):
     sc = make_scene(60011, 2e6, seed=4, targets=[Target(25, 300.0, -40.0)])
     ok, y = D.wienerhopf_process(sc.x, sc.y, -10, 60)
+    assert ok and bool(gold["wh_ok"]) and max(fixture_errors(y, gold, "wh_y")) < 1e-9
     ok_ref, y_ref = (R.wienerhopf_process if R.available() else O.wienerhopf_process)(sc.x, sc.y, -10, 60)
     assert ok and ok_ref
     assert relerr(y, y_ref)[0] < 1e-9
@@ -67,7 +81,7 @@ def test_wienerhopf_class_matches_reference_class(D, relerr):
     assert not ok and np.array_equal(y, np.ones(2048))
 
 
-def test_whole_loop_body_with_dropin_classes(D, relerr):
+def test_whole_loop_body_with_dropin_classes(D, relerr, gold):
     """src/blah2.cpp:268-287 through the class API: filter -> ambiguity -> set_metrics (the reference's
     own Map code) -> CFAR -> Centroid -> Interpolate."""
     # geometry inside the reference's own valid domain: its Doppler work buffer has nfft entries but the
@@ -78,6 +92,13 @@ def test_whole_loop_body_with_dropin_classes(D, relerr):
                 clutter=(-10, 60), pfa=1e-5, nGuard=2, nTrain=6, minDelay=5, minDoppler=15.0, nCentroid=6)
     sc = make_scene(n, fs, seed=5, targets=[Target(37, 600.0, -30.0), Target(92, -400.0, -35.0)])
     d = D.Chain(**args).run(sc.x, sc.y)
+    assert not d["skipped"]
+    e = fixture_errors(d["map"], gold, "chain_map")
+    assert max(e) < 1e-5, e
+    assert abs(d["noisePower"] - float(gold["chain_metrics"][0])) < 1e-3
+    assert len(d["detections"][0]) == gold["chain_detections"].shape[1] >= 2
+    for a, b in zip(d["detections"], gold["chain_detections"]):
+        assert np.max(np.abs(a - b)) < 1e-2
     if R.available():
         r = R.Chain(**args).run(sc.x, sc.y)
         ref_map, ref_det, noise = r["map"], r["detections"], r["noisePower"]
